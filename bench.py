@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- diffusion steps/sec of the PoseDiffusion sampling hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg3|cfg1|cfg2|cfg4|cfg5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg3|cfg1|cfg2|cfg4|cfg5] [--dump-outputs DIR]
     (N > 1: launched by torchrun, one rank per GPU over NCCL)
 
 A bench "step" is one full p_sample_loop of the workload: T = 100 diffusion steps of one 20-frame sequence per GPU,
@@ -44,6 +44,23 @@ WORKLOADS = {
 FEATURES_DESC = ("widened row SURVEY 8f-2 (NOT the headline): MultiScaleImageFeatureExtractor = DINO ViT-S/16 at scales 1, 1/2, 1/3 over "
                  "20 frames of 224x224 per sequence (264 tokens per frame), the stage that produces z for the sampler")
 ALGO_BYTES_PER_MATCH_EVAL = 16  # kp1.xy + kp2.xy as fp32 (SURVEY.md §8d)
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, arrays: dict):
+    """--dump-outputs: what the timed path returned in its last step, one float32 DIR/<name>.npy per array, so that two builds can
+    be compared output for output on the same seeded inputs.  Above DUMP_LIMIT_BYTES in all, every array keeps a fixed, seeded
+    sample of the rows along its first axis.  GGS-off workloads repeat to within 1e-6 of max|pose|; with GGS on, the float
+    atomics of the GGS kernel's shared-memory sums change the order of additions from run to run, and the guided steps amplify
+    that: two runs of one build differed by up to 2 % of max|pose| at cfg3 (1x B200, 1000 W power limit)."""
+    os.makedirs(directory, exist_ok=True)
+    total = sum(t.numel() * 4 for t in arrays.values())
+    for name, t in arrays.items():
+        a = t.detach().to(torch.float32).cpu().numpy()
+        if total > DUMP_LIMIT_BYTES:
+            keep = max(1, a.shape[0] * DUMP_LIMIT_BYTES // total)
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(directory, f"{name}.npy"), a)
 
 
 def read_peaks():
@@ -97,9 +114,9 @@ class ClockSampler:
 
 
 # ----------------------------------------------------------------------------------------------------
-# CPU arm.  The reference is Python: its unmodified `models` / `util` packages are imported from /root/reference (build
-# container) or from baseline/_ref (installed by oracle/install_reference.py; what the GPU box has) behind the pytorch3d /
-# hydra shim of oracle/shims -> kind "reference".  If neither exists the oracle port (oracle/pose_oracle.py, the same operator
+# CPU arm.  The reference is Python: its unmodified `models` / `util` packages are imported from the reference checkout or
+# from oracle/_ref (installed there by oracle/install_reference.py during build()) behind the pytorch3d / hydra shim of
+# oracle/shims -> kind "reference".  If neither exists the oracle port (oracle/pose_oracle.py, the same operator
 # sequence restated) is timed instead -> kind "port".  Bounded sample, extrapolated to the full loop.
 # ----------------------------------------------------------------------------------------------------
 def host_thread_candidates():
@@ -310,6 +327,8 @@ def features_main(args):
     if not args.no_cpu_baseline and world == 1:
         res = cpu_features_run(96, args.seed, min(os.cpu_count() or 1, 32))
         line["cpu_baseline"] = {"value": res["images_per_s"], "unit": "images/s", "cores": res["threads"], "kind": "port", "sample": res["sample"]}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"z": z})
     print(json.dumps(line))
     if world > 1:
         torch.distributed.destroy_process_group()
@@ -331,7 +350,12 @@ def main():
                     help="HBM layout of the packed match stream (csrc/ggs_layout.cuh); 'paired' is the library default, see DESIGN.md 4.1")
     ap.add_argument("--denoiser-engine", default="auto", choices=["auto", "fp32", "tf32"],
                     help="auto = exact-fp32 persistent kernel below 128 tokens per GPU, tcgen05/TMA tiles (TF32) at or above")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (the gathered poses; z of rank 0 for --workload "
+                         "features) as DIR/<name>.npy in float32")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200: the reference arm times a bounded sample and computes no complete output")
     if args.seqs_per_gpu is None:
         args.seqs_per_gpu = 8 if args.workload == "cfg4" else 1
     if args.workload == "features":
@@ -522,6 +546,8 @@ def main():
         res = cpu_reference_run(frames, per_pair, args.seed, args.cpu_budget)
         line["cpu_baseline"] = {"value": res["steps_per_s"], "unit": "diffusion steps/s", "cores": res["threads"], "kind": res["kind"],
                                 "sample": res["sample"], "wall_s_full_extrapolated": res["wall_s_full"]}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"pose": full})
     print(json.dumps(line))
     if world > 1:
         torch.distributed.destroy_process_group()

@@ -1,8 +1,8 @@
-"""Import the reference's OWN hot-path modules from /root/reference (build container only).
+"""Import the reference's OWN hot-path modules from the reference checkout (POSEDIFF_REFERENCE_ROOT).
 
-TEST INFRASTRUCTURE.  /root/reference does not exist on the GPU box; there the same unmodified modules are imported from
-baseline/_ref (installed by oracle/install_reference.py).  Used by `oracle/make_golden.py` (fixture generation), by CPU tests
-that skip when neither is present, and by `bench.py --impl reference` / the `cpu_baseline` leg.
+TEST INFRASTRUCTURE.  Where the checkout is absent, the same unmodified modules are imported from oracle/_ref (installed
+there by oracle/install_reference.py during `build()`).  Used by `oracle/make_golden.py` (fixture generation) and by
+`bench.py --impl reference` / the `cpu_baseline` leg, which time the oracle port when neither is present.
 pytorch3d and hydra are not installed here; `oracle/shims/` restates the handful of symbols
 the reference imports (SURVEY.md §8c).  Nothing is copied: the modules are imported in place.
 """
@@ -14,9 +14,8 @@ from types import SimpleNamespace
 
 REFERENCE_ROOT = os.environ.get("POSEDIFF_REFERENCE_ROOT", "/root/reference")
 _SHIMS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "shims")
-# the unmodified `models` / `util` packages installed by oracle/install_reference.py (git-ignored; present on the GPU box)
-INSTALLED_ROOT = os.environ.get("POSEDIFF_INSTALLED_REFERENCE",
-                                os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref"))
+# the unmodified `models` / `util` packages installed by oracle/install_reference.py (git-ignored build output)
+INSTALLED_ROOT = os.environ.get("POSEDIFF_INSTALLED_REFERENCE", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 TRANSFORMER_CFG = dict(
     _target_="models.TransformerEncoderWrapper",
@@ -31,8 +30,8 @@ TRANSFORMER_CFG = dict(
 
 
 def reference_path() -> str | None:
-    """Directory that holds the reference's `models` and `util` packages: the source tree in the build container, else the
-    copy installed into baseline/_ref (what the GPU box has), else None."""
+    """Directory that holds the reference's `models` and `util` packages: the reference checkout when present, else the
+    copy installed into oracle/_ref, else None."""
     src = os.path.join(REFERENCE_ROOT, "pose_diffusion")
     if os.path.isdir(os.path.join(src, "models")):
         return src

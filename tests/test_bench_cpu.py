@@ -1,6 +1,7 @@
-"""CPU-only checks of bench.py's contract: the reference arm (`--impl reference`: the reference's own modules from /root/reference
-or baseline/_ref when present, else the CPU oracle port, on the host cores) prints ONE JSON line with the keys the driver reads, non-zero ranks of a multi-process launch exit without work, and the b200 arm
-refuses to run without a GPU instead of falling back."""
+"""CPU-only checks of bench.py's output contract: the reference arm (`--impl reference`: the reference's own modules from the
+reference checkout or oracle/_ref when present, else the CPU oracle port, on the host cores) prints ONE JSON line with the
+documented keys, non-zero ranks of a multi-process launch exit without work, and the b200 arm refuses to run without a GPU
+instead of falling back."""
 import json
 import os
 import subprocess
@@ -38,7 +39,7 @@ def test_reference_arm_prints_one_contract_line():
 
 
 def test_reference_arm_falls_back_to_the_port_without_the_reference(tmp_path):
-    """Neither /root/reference nor baseline/_ref: the arm times the oracle port and says so (`kind: "port"`)."""
+    """Neither the reference checkout nor oracle/_ref: the arm times the oracle port and says so (`kind: "port"`)."""
     res = run(["--impl", "reference", "--workload", "cfg1", "--gpus", "1", "--steps", "1", "--warmup", "1"],
               env={"POSEDIFF_REFERENCE_ROOT": str(tmp_path), "POSEDIFF_INSTALLED_REFERENCE": str(tmp_path)})
     assert res.returncode == 0, res.stderr[-2000:]
@@ -59,6 +60,13 @@ def test_reference_arm_other_ranks_exit_without_work():
     res = run(["--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "1"], env={"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"},
               timeout=120)
     assert res.returncode == 0 and res.stdout.strip() == ""
+
+
+def test_reference_arm_refuses_dump_outputs(tmp_path):
+    """The reference arm extrapolates from a bounded sample, so it has no complete output to dump."""
+    res = run(["--impl", "reference", "--steps", "1", "--dump-outputs", str(tmp_path / "out")], timeout=120)
+    assert res.returncode != 0 and "--dump-outputs" in res.stderr
+    assert not (tmp_path / "out").exists()
 
 
 def test_b200_arm_has_no_cpu_fallback():
